@@ -5,10 +5,14 @@ BIGINT key), plus the Q1 GROUP-BY input rows/s, through the C ABI of libtrino_gp
   python bench.py --gpus 1 --steps K --warmup W            # this repo's sm_100a operators
   python bench.py --impl reference --gpus N ...            # the reference's CPU algorithm (C++ restatement, all host threads)
   torchrun ... bench.py --gpus N ...                       # partitioned join: hash exchange over NCCL + local probe
+  python bench.py --gpus 1 ... --dump-outputs DIR          # also write the joined page of the last timed step to DIR/*.npy
 
 A "step" is one pass of the LookupJoinOperator over the whole probe side (N>1: PagePartitioner + all-to-all + probe).
 `value` is timed with inputs resident in HBM; `e2e` feeds HOST pages through the same operator calls and copies the
 result back to host memory inside the timed region.  Prints ONE JSON line on rank 0.
+
+The inputs are generated from fixed seeds, so two builds run with the same arguments join the same rows, and their
+--dump-outputs directories can be compared file by file.
 """
 import argparse
 import ctypes as C
@@ -22,10 +26,14 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
+sys.dont_write_bytecode = True      # the benchmark leaves the tree it runs from as it found it (it may be read-only)
 
 import numpy as np  # noqa: E402
 
 SEED_LINEITEM, SEED_ORDERS = 0x7C01, 0x7C02
+# --dump-outputs: a joined page of more rows than this is written as DUMP_RUNS runs of DUMP_RUN_ROWS consecutive rows at
+# places drawn with SEED_DUMP (4 files x 8 MB of float64 at most)
+DUMP_RUNS, DUMP_RUN_ROWS, SEED_DUMP = 512, 2048, 0x7C0D
 ALG_BYTES_PROBE_INDEX = 24          # SURVEY.md §8d: 8 key + 12 table entry + 4 position
 ALG_BYTES_PROBE_FUSED = 40          # fused probe + gather, this workload: 24 + 8 build payload read + 8 written (probe columns pass through by reference)
 ALG_BYTES_Q1_CODES = 38             # shipdate 4 + 4 x FLOAT64 32 + 2 INT8 key codes
@@ -142,7 +150,7 @@ def cpu_probe_measure(args, n_orders, probe_rows, passes, warm):
     pay = pj.alloc(sample, np.int32)
     for _ in range(max(1, warm)):
         pj.probe(lkeys, pos, pay)
-    times = sorted(pj.probe(lkeys, pos, pay) for _ in range(max(passes, 10)))
+    times = sorted(pj.probe(lkeys, pos, pay) for _ in range(passes))
     assert (pos >= 0).all()
     assert (pay[:4096] == (lkeys[:4096] % 2557)).all()
     med = float(np.median(times))
@@ -192,6 +200,28 @@ def device_col(ctx, nbytes):
     return ctx.malloc(nbytes)
 
 
+def dump_page(ctx, out, names, path):
+    """Write the columns of a device output page as path/<name>.npy in float64 (the BIGINT values here stay below 2^53), with
+    path/row.npy = the positions in the page of the rows written: every row of a small page, else the seeded sample of
+    DUMP_RUNS runs of DUMP_RUN_ROWS rows, which is the same for every page of the same row count."""
+    from trino_b200 import abi
+    n = out.rows
+    if n <= DUMP_RUNS * DUMP_RUN_ROWS:
+        runs = [(0, n)]
+    else:
+        starts = np.sort(np.random.default_rng(SEED_DUMP).choice(n // DUMP_RUN_ROWS, DUMP_RUNS, replace=False)) * DUMP_RUN_ROWS
+        runs = [(int(s), DUMP_RUN_ROWS) for s in starts]
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "row.npy"), np.concatenate([np.arange(s, s + m, dtype=np.float64) for s, m in runs]))
+    dtypes = {abi.INT64: np.dtype(np.int64), abi.FLOAT64: np.dtype(np.float64)}
+    for c, name in enumerate(names):
+        col = out.column(c)
+        assert not col.validity, f"{name}: NULLs are not written"
+        dt = dtypes[col.type]
+        vals = np.concatenate([ctx.to_host(col.ptr + s * dt.itemsize, dt, m) for s, m in runs])
+        np.save(os.path.join(path, name + ".npy"), vals.astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -213,7 +243,14 @@ def main():
     ap.add_argument("--no-secondary", action="store_true", help="skip the FilterAndProject / PartitionedOutput blocks (secondary_operators)")
     ap.add_argument("--no-e2e", action="store_true", help="skip the end-to-end (host pages) measurement: kernel experiments only")
     ap.add_argument("--l2-fetch", type=int, default=0, help="cudaLimitMaxL2FetchGranularity to set (32/64/128; 0 = leave the default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the joined page of the last one as DIR/<column>.npy (float64; a fixed seeded sample of "
+                         f"{DUMP_RUNS} x {DUMP_RUN_ROWS} rows of a larger page, DIR/row.npy = their positions in the page)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.impl != "b200" or args.workload != "join" or dist_env()[1] > 1):
+        ap.error("--dump-outputs is implemented for the join workload of --impl b200 on one GPU")
     if args.sf is None:
         args.sf = 37.5 if args.workload == "q3way" else 100.0
     if args.impl == "reference":
@@ -390,7 +427,9 @@ def main():
         probe_op.add_input(inp.as_device_page())
         inflight.append(inp)
 
-    def step():
+    last_out = [None]
+
+    def step(keep_output=False):
         if overlap:
             step_overlapped()
         elif partitioner is not None:
@@ -411,7 +450,10 @@ def main():
             out = probe_op.get_output_device()
             out_rows_seen[0] = out.rows if out else 0
             if out:
-                out.release()
+                if keep_output:
+                    last_out[0] = out          # --dump-outputs: written and released after the timed region
+                else:
+                    out.release()
 
     for _ in range(args.warmup):
         step()
@@ -427,8 +469,8 @@ def main():
     step_rows[0] = 0
     launches0 = ctx.kernel_launches + 0
     ctx.timer_start()
-    for _ in range(args.steps):
-        step()
+    for i in range(args.steps):
+        step(keep_output=args.dump_outputs is not None and i == args.steps - 1)
     if overlap:
         # pipeline drain: the last exchange is ended and probed, its output taken (host-synchronised) before the stop event
         while handles:
@@ -438,6 +480,10 @@ def main():
     ms = ctx.timer_stop_ms()
     launches = ctx.kernel_launches + 0 - launches0
     clocks = sampler.stop()
+    if args.dump_outputs is not None:
+        assert last_out[0] is not None, "the last timed step produced no page"
+        dump_page(ctx, last_out[0], ["l_orderkey", "l_extendedprice", "o_orderdate"], args.dump_outputs)
+        last_out[0].release()
     barrier()
     if dist is not None:
         import torch
