@@ -252,16 +252,30 @@ struct GatherCols {
     void* dst[4];
 };
 
+// Match bitmap of the fused probe kernels: LSB first, bit i = probe row i matched - the Arrow validity layout, so a PROBE_OUTER join hands
+// it to the build columns as it is.  Every fused kernel runs 256-thread CTAs over 1024-row tiles, where the j-th row set of a warp (rows
+// tile * 1024 + j * 256 + 32 * warp + lane) is 32 consecutive rows: one ballot, one word written by lane 0.  Every lane of the warp must
+// call it (a lane without a row votes false).  Returns the number of matches of the word on lane 0, 0 on the other lanes.
+__device__ __forceinline__ unsigned int match_bits_word(unsigned int* __restrict__ bits, int64_t tile, int j, bool hit)
+{
+    const unsigned int w = __ballot_sync(0xffffffffu, hit);
+    if ((threadIdx.x & 31) != 0) return 0;
+    bits[tile * 32 + j * 8 + (threadIdx.x >> 5)] = w;
+    return __popc(w);
+}
+
 // Fused probe + build-side gather for the common join shape (no duplicate chains, fixed-width non-null build
 // columns): the chain head is looked up and the build payload of the matching row is fetched while the slot is
 // still in flight in the same thread, so the positions never make a round trip through HBM before the gather and
-// no count/scan pass is needed when every probe row matches (FK -> PK joins).  Misses are counted; the host
-// compacts only when there are any.
-template <int ROWS, bool INT64_NO_NULLS>
+// no count/scan pass is needed when every probe row matches (FK -> PK joins).  Misses are counted and marked in the
+// match bitmap; the host compacts only when there are any.
+template <bool INT64_NO_NULLS>
 __global__ void __launch_bounds__(256) join_probe_gather_kernel(ColRef key, int kind, int64_t n, const JoinSlot* __restrict__ table, JoinGeom geo,
-                                                                int special_head, int* __restrict__ out, GatherCols g, unsigned long long* __restrict__ match_count)
+                                                                int special_head, GatherCols g, unsigned int* __restrict__ match_bits,
+                                                                unsigned long long* __restrict__ match_count)
 {
     // g.by_slot: payload arrays are indexed by table slot (special key at index mask + 1), else by build row id
+    constexpr int ROWS = 4;      // 256 threads x 4 rows: the 1024-row tiles of match_bits_word
     int64_t tile = (int64_t)blockDim.x * ROWS;
     int64_t tiles = (n + tile - 1) / tile;
     unsigned int matched = 0;
@@ -337,43 +351,19 @@ __global__ void __launch_bounds__(256) join_probe_gather_kernel(ColRef key, int 
                 }
             }
         }
+        // rows past n have res = -1 and vote 0; every lane reaches the ballot
 #pragma unroll
-        for (int j = 0; j < ROWS; j++) {
-            int64_t i = base + (int64_t)j * blockDim.x;
-            if (i >= n) continue;
-            out[i] = res[j];
-            matched += res[j] >= 0;
-        }
+        for (int j = 0; j < ROWS; j++) matched += match_bits_word(match_bits, t, j, res[j] >= 0);
     }
     // one atomic per warp
-    for (int off = 16; off > 0; off >>= 1) matched += __shfl_xor_sync(0xffffffffu, matched, off);
     if ((threadIdx.x & 31) == 0 && matched) atomicAdd(match_count, (unsigned long long)matched);
 }
 
-// validity bitmap of the build side of a PROBE_OUTER join: bit i = (jp[i] >= 0)
-__global__ void join_match_validity_kernel(const int* __restrict__ jp, int64_t n, uint8_t* __restrict__ bitmap)
-{
-    int64_t b = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    int64_t nbytes = (n + 7) >> 3;
-    int64_t stride = (int64_t)gridDim.x * blockDim.x;
-    for (; b < nbytes; b += stride) {
-        unsigned int v = 0;
-        int64_t base = b << 3;
-#pragma unroll
-        for (int k = 0; k < 8; k++) {
-            int64_t i = base + k;
-            if (i < n && jp[i] >= 0) v |= 1u << k;
-        }
-        bitmap[b] = (uint8_t)v;
-    }
-}
-
-__global__ void join_match_flags_kernel(const int* __restrict__ jp, int64_t n, uint8_t* __restrict__ flags)
-{
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    int64_t stride = (int64_t)gridDim.x * blockDim.x;
-    for (; i < n; i += stride) flags[i] = jp[i] >= 0 ? 1 : 0;
-}
+// select predicate over row numbers: bit i of the match bitmap
+struct MatchBit {
+    const unsigned int* bits;
+    __device__ __forceinline__ bool operator()(int32_t i) const { return (bits[i >> 5] >> (i & 31)) & 1u; }
+};
 
 
 
@@ -469,9 +459,11 @@ static int lean_grid(tgpu_ctx* ctx, K kernel, int64_t tiles)
     return (int)std::min<int64_t>(tiles, (int64_t)ctx->sm_count * per_sm);
 }
 
+// GATHER: the payload columns of g are written and, instead of positions, a match bitmap (see match_bits_word); else out = positions
 template <int MODE, bool GATHER, int MINB = 1>
 __global__ void __launch_bounds__(256, MINB) join_probe_lean_kernel(const long long* __restrict__ keys, int64_t tiles, const int4* __restrict__ table, unsigned int mask,
-                                                              unsigned long long kmin, int shift, int special_head, int* __restrict__ out, GatherCols g, unsigned long long* __restrict__ match_count)
+                                                              unsigned long long kmin, int shift, int special_head, int* __restrict__ out, GatherCols g,
+                                                              unsigned int* __restrict__ match_bits, unsigned long long* __restrict__ match_count)
 {
     // the word behind the match counter holds the layout choice of the page (0 = these 16-byte slots; join_probe_locality_kernel decides)
     if (GATHER && *(const volatile int*)(match_count + 1) != 0) return;
@@ -534,195 +526,31 @@ __global__ void __launch_bounds__(256, MINB) join_probe_lean_kernel(const long l
         }
 #pragma unroll
         for (int j = 0; j < 4; j++) {
-            out[base + j * 256] = res[j];
-            if (GATHER) matched += res[j] >= 0;
+            if (GATHER) matched += match_bits_word(match_bits, t, j, res[j] >= 0);
+            else out[base + j * 256] = res[j];
         }
     }
-    if (GATHER) {
-        for (int off = 16; off > 0; off >>= 1) matched += __shfl_xor_sync(0xffffffffu, matched, off);
-        if ((threadIdx.x & 31) == 0 && matched) atomicAdd(match_count, (unsigned long long)matched);
-    }
-}
-
-// ---- TMA-staged probe for order-preserving tables (mode 2) ----------------------------------------------------------------
-// With order-preserving lines a tile of probe keys that arrives in key order (TPC-H clustering; each sender's run after a stable
-// exchange) needs ONE contiguous span of table lines.  The CTA computes the span of its 1024 keys, one elected thread stages the span -
-// the 16-byte slots and, for the common single-BIGINT-payload shape, the slot-ordered payload next to them - into shared memory with
-// cp.async.bulk (TMA bulk copy, completion on an mbarrier), and every thread then resolves its four rows against shared memory:
-// one bulk copy of full 128-byte lines replaces ~2 x 1024 scattered 16 / 8-byte loads.  A tile whose span does not fit (shuffled keys, keys
-// outside the build range) takes the direct path of the lean kernel; a row whose line walk leaves the staged span falls back to global
-// loads for its remaining steps.
-constexpr int SPAN_LINES = 80;            // table lines staged per tile: 10 KB of slots + 5 KB of payload
-
-__device__ __forceinline__ unsigned int smem_u32(const void* p) { return (unsigned int)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, int count)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, unsigned int bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_gmem, unsigned int bytes, unsigned long long* bar)
-{
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst_smem)), "l"(src_gmem), "r"(bytes),
-                 "r"(smem_u32(bar))
-                 : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned int parity)
-{
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "TG_WAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra TG_DONE_%=;\n"
-        "bra TG_WAIT_%=;\n"
-        "TG_DONE_%=:\n"
-        "}\n" ::"r"(smem_u32(bar)),
-        "r"(parity)
-        : "memory");
-}
-
-template <bool GATHER>
-__global__ void __launch_bounds__(256, 6) join_probe_span_kernel(const long long* __restrict__ keys, int64_t tiles, const int4* __restrict__ table, unsigned int mask,
-                                                                unsigned long long kmin, int shift, int special_head, int* __restrict__ out, GatherCols g,
-                                                                unsigned long long* __restrict__ match_count)
-{
-    __shared__ __align__(128) int4 s_slots[SPAN_LINES * 8];
-    __shared__ __align__(128) long long s_pay[SPAN_LINES * 8];
-    __shared__ __align__(8) unsigned long long bar;
-    __shared__ unsigned int s_min[8], s_max[8];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const unsigned int line_mask = mask >> 3;
-    // the slot-ordered single 8-byte payload is staged next to the slots; other payload shapes are read from global memory
-    const bool stage_pay = GATHER && g.by_slot && g.count == 1 && g.elem[0] == 8;
-    if (threadIdx.x == 0) mbar_init(&bar, 1);
-    __syncthreads();
-    unsigned int phase = 0;
-    unsigned int matched = 0;
-    for (int64_t t = blockIdx.x; t < tiles; t += gridDim.x) {
-        const int64_t base = t * 1024 + threadIdx.x;
-        unsigned long long k[4];
-        unsigned int pos[4];
-#pragma unroll
-        for (int j = 0; j < 4; j++) k[j] = (unsigned long long)__ldg(keys + base + j * 256);
-        unsigned int lo = 0xffffffffu, hi = 0;
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-            pos[j] = lean_slot<2>(k[j], mask, kmin, shift);
-            const unsigned int line = pos[j] >> 3;
-            lo = min(lo, line);
-            hi = max(hi, line);
-        }
-        lo = __reduce_min_sync(0xffffffffu, lo);
-        hi = __reduce_max_sync(0xffffffffu, hi);
-        if (lane == 0) { s_min[warp] = lo; s_max[warp] = hi; }
-        __syncthreads();
-#pragma unroll
-        for (int w = 0; w < 8; w++) { lo = min(lo, s_min[w]); hi = max(hi, s_max[w]); }
-        // one extra line behind the span for line walks that overflow their home line
-        const unsigned int first_line = lo, lines = min(hi + 1u, line_mask) - lo + 1u;
-        const bool staged = lines <= (unsigned int)SPAN_LINES;
-        if (staged) {
-            if (threadIdx.x == 0) {
-                const unsigned int slot_bytes = lines * 128u, pay_bytes = stage_pay ? lines * 64u : 0u;
-                mbar_expect_tx(&bar, slot_bytes + pay_bytes);
-                bulk_g2s(s_slots, table + (size_t)first_line * 8, slot_bytes, &bar);
-                if (stage_pay) bulk_g2s(s_pay, (const long long*)g.src[0] + (size_t)first_line * 8, pay_bytes, &bar);
-            }
-            mbar_wait(&bar, phase);
-            phase ^= 1u;
-        }
-        const unsigned int first_slot = first_line << 3, staged_slots = staged ? lines << 3 : 0u;
-        int res[4];
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-            const unsigned int klo = (unsigned int)k[j], khi = (unsigned int)(k[j] >> 32);
-            int r = -1;
-            unsigned int p = pos[j];
-            while (true) {
-                const unsigned int local = p - first_slot;
-                const int4 cur = local < staged_slots ? s_slots[local] : __ldg(table + p);
-                if ((unsigned int)cur.x == klo && (unsigned int)cur.y == khi) { r = cur.z; break; }
-                if (cur.x == 0 && cur.y == (int)0x80000000) break;                 // EMPTY_KEY
-                p = lean_next<2>(p, klo & 7u, mask);
-            }
-            if (k[j] == EMPTY_KEY) { r = special_head; p = mask + 1u; }
-            res[j] = r;
-            pos[j] = p;
-        }
-        if (GATHER) {
-#pragma unroll
-            for (int c = 0; c < 4; c++) {
-                if (c >= g.count) break;
-                if (g.elem[c] == 8) {
-                    long long v[4];
-#pragma unroll
-                    for (int j = 0; j < 4; j++) {
-                        const unsigned int local = pos[j] - first_slot;
-                        if (res[j] < 0) v[j] = 0;
-                        else if (stage_pay && local < staged_slots) v[j] = s_pay[local];
-                        else v[j] = __ldg((const long long*)g.src[c] + (g.by_slot ? (long long)pos[j] : (long long)res[j]));
-                    }
-#pragma unroll
-                    for (int j = 0; j < 4; j++) ((long long*)g.dst[c])[base + j * 256] = v[j];
-                }
-                else if (g.elem[c] == 4) {
-#pragma unroll
-                    for (int j = 0; j < 4; j++)
-                        ((int*)g.dst[c])[base + j * 256] = res[j] >= 0 ? __ldg((const int*)g.src[c] + (g.by_slot ? (long long)pos[j] : (long long)res[j])) : 0;
-                }
-                else {
-#pragma unroll
-                    for (int j = 0; j < 4; j++) {
-                        long long at = g.by_slot ? (long long)pos[j] : (long long)res[j];
-                        if (g.elem[c] == 2) ((short*)g.dst[c])[base + j * 256] = res[j] >= 0 ? ((const short*)g.src[c])[at] : (short)0;
-                        else ((signed char*)g.dst[c])[base + j * 256] = res[j] >= 0 ? ((const signed char*)g.src[c])[at] : (signed char)0;
-                    }
-                }
-            }
-        }
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-            out[base + j * 256] = res[j];
-            if (GATHER) matched += res[j] >= 0;
-        }
-        __syncthreads();          // everyone is done with the staged span (and s_min / s_max) before the next tile overwrites them
-    }
-    if (GATHER) {
-        for (int off = 16; off > 0; off >>= 1) matched += __shfl_xor_sync(0xffffffffu, matched, off);
-        if (lane == 0 && matched) atomicAdd(match_count, (unsigned long long)matched);
-    }
+    if (GATHER && (threadIdx.x & 31) == 0 && matched) atomicAdd(match_count, (unsigned long long)matched);
 }
 
 // launch of the lean probe kernel for the table's layout mode
 template <bool GATHER>
 static int launch_lean(tgpu_ctx* ctx, const JoinGeom& geo, const long long* keys, int64_t tiles, const int4* table, int special_head, int* out, const GatherCols& g,
-                       unsigned long long* matches)
+                       unsigned int* match_bits, unsigned long long* matches)
 {
     const unsigned int mask32 = (unsigned int)geo.mask;
     // 8 CTAs per SM (32 registers): full occupancy is worth more than the registers (measured 4.9 -> 3.4 ms at SF100)
-    if (geo.mode == 2 && getenv("TGPU_JOIN_SPAN")) {
-        // TMA-staged table spans (falls back per tile when the keys are not clustered).  Opt-in: measured 9 % SLOWER than the lean kernel on
-        // the SF100 workload (2.73 vs 2.50 ms) - with the dense table the lean kernel already moves its 15.6 GB at 0.95 of the measured copy
-        // bandwidth, and the span kernel pays a block-wide span reduction plus a second dependent DRAM round trip per tile
-        auto k = join_probe_span_kernel<GATHER>;
-        TG_LAUNCH(ctx, k, lean_grid(ctx, k, tiles), 256, 0, keys, tiles, table, mask32, geo.kmin, geo.shift, special_head, out, g, matches);
-    }
-    else if (geo.mode == 2) {
+    if (geo.mode == 2) {
         auto k = join_probe_lean_kernel<2, GATHER, 8>;
-        TG_LAUNCH(ctx, k, lean_grid(ctx, k, tiles), 256, 0, keys, tiles, table, mask32, geo.kmin, geo.shift, special_head, out, g, matches);
+        TG_LAUNCH(ctx, k, lean_grid(ctx, k, tiles), 256, 0, keys, tiles, table, mask32, geo.kmin, geo.shift, special_head, out, g, match_bits, matches);
     }
     else if (geo.mode == 1) {
         auto k = join_probe_lean_kernel<1, GATHER, 8>;
-        TG_LAUNCH(ctx, k, lean_grid(ctx, k, tiles), 256, 0, keys, tiles, table, mask32, 0ULL, 0, special_head, out, g, matches);
+        TG_LAUNCH(ctx, k, lean_grid(ctx, k, tiles), 256, 0, keys, tiles, table, mask32, 0ULL, 0, special_head, out, g, match_bits, matches);
     }
     else {
         auto k = join_probe_lean_kernel<0, GATHER, 8>;
-        TG_LAUNCH(ctx, k, lean_grid(ctx, k, tiles), 256, 0, keys, tiles, table, mask32, 0ULL, 0, special_head, out, g, matches);
+        TG_LAUNCH(ctx, k, lean_grid(ctx, k, tiles), 256, 0, keys, tiles, table, mask32, 0ULL, 0, special_head, out, g, match_bits, matches);
     }
     return TGPU_OK;
 }
@@ -788,7 +616,7 @@ __global__ void join_wide_table_kernel(const JoinSlot* __restrict__ table, int64
 // flight together (a tile is 4 rows per thread, taken ROWS at a time)
 template <int MODE, int ROWS, int MINB, int LD = 0>
 __global__ void __launch_bounds__(256, MINB) join_probe_wide_kernel(const long long* __restrict__ keys, int64_t tiles, const WideSlot* __restrict__ wide, unsigned int mask,
-                                                                  unsigned long long kmin, int shift, int special_head, int* __restrict__ out, GatherCols g,
+                                                                  unsigned long long kmin, int shift, int special_head, GatherCols g, unsigned int* __restrict__ match_bits,
                                                                   unsigned long long* __restrict__ match_count, const int* __restrict__ layout_choice)
 {
     if (layout_choice && *layout_choice == 0) return;      // the page goes through the 16-byte slots
@@ -838,18 +666,14 @@ __global__ void __launch_bounds__(256, MINB) join_probe_wide_kernel(const long l
                 }
             }
 #pragma unroll
-            for (int j = 0; j < ROWS; j++) {
-                out[base + j * 256] = w[j].head;
-                matched += w[j].head >= 0;
-            }
+            for (int j = 0; j < ROWS; j++) matched += match_bits_word(match_bits, t, h + j, w[j].head >= 0);
         }
     }
-    for (int off = 16; off > 0; off >>= 1) matched += __shfl_xor_sync(0xffffffffu, matched, off);
     if ((threadIdx.x & 31) == 0 && matched) atomicAdd(match_count, (unsigned long long)matched);
 }
 
 // Which layout a probe page should read.  A wide slot is 32 bytes, a 16-byte slot plus its slot-ordered payload cells 16 + (payload bytes):
-// with one payload column a probe page that arrives in key order reads fewer bytes from the narrow layout (whole lines are used either
+// with less than 16 bytes of payload a probe page that arrives in key order reads fewer bytes from the narrow layout (whole lines are used either
 // way), while a page without key locality pays a 32-byte sector per ARRAY it touches and is better off with the wide slot.  256 pairs of
 // neighbouring rows, spread over the page, vote: a pair is local when its two slots lie within 8 lines of each other.
 // choice: 0 = narrow, 1 = wide.  No host round trip: both probe kernels are launched and the one not chosen returns at once.
@@ -875,42 +699,133 @@ static int launch_locality(tgpu_ctx* ctx, const JoinGeom& geo, const long long* 
 }
 
 template <int ROWS, int MINB, int LD = 0>
-static int launch_wide_shape(tgpu_ctx* ctx, const JoinGeom& geo, const long long* keys, int64_t tiles, const WideSlot* wide, int special_head, int* out,
-                             const GatherCols& g, unsigned long long* matches, const int* layout_choice)
+static int launch_wide_shape(tgpu_ctx* ctx, const JoinGeom& geo, const long long* keys, int64_t tiles, const WideSlot* wide, int special_head, const GatherCols& g,
+                             unsigned int* match_bits, unsigned long long* matches, const int* layout_choice)
 {
     const unsigned int mask32 = (unsigned int)geo.mask;
     if (geo.mode == 2) {
         auto k = join_probe_wide_kernel<2, ROWS, MINB, LD>;
-        TG_LAUNCH(ctx, k, lean_grid(ctx, k, tiles), 256, 0, keys, tiles, wide, mask32, geo.kmin, geo.shift, special_head, out, g, matches, layout_choice);
+        TG_LAUNCH(ctx, k, lean_grid(ctx, k, tiles), 256, 0, keys, tiles, wide, mask32, geo.kmin, geo.shift, special_head, g, match_bits, matches, layout_choice);
     }
     else if (geo.mode == 1) {
         auto k = join_probe_wide_kernel<1, ROWS, MINB, LD>;
-        TG_LAUNCH(ctx, k, lean_grid(ctx, k, tiles), 256, 0, keys, tiles, wide, mask32, 0ULL, 0, special_head, out, g, matches, layout_choice);
+        TG_LAUNCH(ctx, k, lean_grid(ctx, k, tiles), 256, 0, keys, tiles, wide, mask32, 0ULL, 0, special_head, g, match_bits, matches, layout_choice);
     }
     else {
         auto k = join_probe_wide_kernel<0, ROWS, MINB, LD>;
-        TG_LAUNCH(ctx, k, lean_grid(ctx, k, tiles), 256, 0, keys, tiles, wide, mask32, 0ULL, 0, special_head, out, g, matches, layout_choice);
+        TG_LAUNCH(ctx, k, lean_grid(ctx, k, tiles), 256, 0, keys, tiles, wide, mask32, 0ULL, 0, special_head, g, match_bits, matches, layout_choice);
     }
     return TGPU_OK;
 }
 
 // rows in flight per thread x CTAs per SM; TGPU_JOIN_WIDE_SHAPE=<rows><ctas> picks one of the built shapes (sweeps)
-static int launch_wide(tgpu_ctx* ctx, const JoinGeom& geo, const long long* keys, int64_t tiles, const WideSlot* wide, int special_head, int* out, const GatherCols& g,
-                       unsigned long long* matches, const int* layout_choice)
+static int launch_wide(tgpu_ctx* ctx, const JoinGeom& geo, const long long* keys, int64_t tiles, const WideSlot* wide, int special_head, const GatherCols& g,
+                       unsigned int* match_bits, unsigned long long* matches, const int* layout_choice)
 {
     const char* e = getenv("TGPU_JOIN_WIDE_SHAPE");
     int shape = e ? atoi(e) : 28;
     const char* le = getenv("TGPU_JOIN_WIDE_LOAD");
     int ld = le ? atoi(le) : 3;       // measured on the shuffled SF100 probe: 0 -> 17.87 ms, 3 -> 17.37 ms, 5 -> 19.5 ms
-    if (shape == 28 && ld == 3) return launch_wide_shape<2, 8, 3>(ctx, geo, keys, tiles, wide, special_head, out, g, matches, layout_choice);
-    if (shape == 28 && ld == 5) return launch_wide_shape<2, 8, 5>(ctx, geo, keys, tiles, wide, special_head, out, g, matches, layout_choice);
+    if (shape == 28 && ld == 3) return launch_wide_shape<2, 8, 3>(ctx, geo, keys, tiles, wide, special_head, g, match_bits, matches, layout_choice);
+    if (shape == 28 && ld == 5) return launch_wide_shape<2, 8, 5>(ctx, geo, keys, tiles, wide, special_head, g, match_bits, matches, layout_choice);
     switch (shape) {
-        case 18: return launch_wide_shape<1, 8>(ctx, geo, keys, tiles, wide, special_head, out, g, matches, layout_choice);
-        case 26: return launch_wide_shape<2, 6>(ctx, geo, keys, tiles, wide, special_head, out, g, matches, layout_choice);
-        case 45: return launch_wide_shape<4, 5>(ctx, geo, keys, tiles, wide, special_head, out, g, matches, layout_choice);
-        case 44: return launch_wide_shape<4, 4>(ctx, geo, keys, tiles, wide, special_head, out, g, matches, layout_choice);
-        default: return launch_wide_shape<2, 8>(ctx, geo, keys, tiles, wide, special_head, out, g, matches, layout_choice);
+        case 18: return launch_wide_shape<1, 8>(ctx, geo, keys, tiles, wide, special_head, g, match_bits, matches, layout_choice);
+        case 26: return launch_wide_shape<2, 6>(ctx, geo, keys, tiles, wide, special_head, g, match_bits, matches, layout_choice);
+        case 45: return launch_wide_shape<4, 5>(ctx, geo, keys, tiles, wide, special_head, g, match_bits, matches, layout_choice);
+        case 44: return launch_wide_shape<4, 4>(ctx, geo, keys, tiles, wide, special_head, g, match_bits, matches, layout_choice);
+        default: return launch_wide_shape<2, 8>(ctx, geo, keys, tiles, wide, special_head, g, match_bits, matches, layout_choice);
     }
+}
+
+// ---- packed slots: key and the head row's payload in ONE 16-byte entry (one-column builds) -----------------------------------------
+// The fused probe needs the head row id only to find the payload.  A build with exactly one fixed-width output column without NULLs and no
+// duplicate keys (the FK -> PK shape of every join in the benchmark) therefore gets a table of {key, payload of the head row zero-extended
+// to 8 bytes} in the slot geometry of the 16-byte table, with entry `capacity` holding the INT64_MIN key's payload under the key EMPTY_KEY.
+// A probe row reads one 16-byte entry - the bytes of the JoinSlot alone - and neither the slot-ordered payload array nor the wide table is
+// built for this shape.  The JoinSlot table stays: the index-only probe, the ragged tail and the generic kernels read it.
+struct __align__(16) PackedSlot {
+    unsigned long long key;
+    unsigned long long cell;
+};
+
+__global__ void join_packed_table_kernel(const JoinSlot* __restrict__ table, int64_t slots, int special_head, const void* __restrict__ src, int elem,
+                                         PackedSlot* __restrict__ packed)
+{
+    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (; i <= slots; i += stride) {
+        const int head = i < slots ? table[i].head : special_head;
+        PackedSlot s;
+        s.key = i < slots ? table[i].key : EMPTY_KEY;
+        s.cell = head >= 0 ? wide_cell_of(src, elem, head) : 0ULL;
+        packed[i] = s;
+    }
+}
+
+// same tile contract as join_probe_lean_kernel<MODE, true>; two rows of a thread are in flight together (a tile is 4 rows per thread,
+// taken 2 at a time): 8 CTAs per SM at 32 registers without spills - with 4 rows the key and entry registers alone take 24 of the 32 and
+// ptxas spills.  special: the key INT64_MIN has a build row.  A miss writes 0 and a 0 bit.  Row numbers are 32-bit (a page has at most
+// 2^31 - 1 rows), and a row's home slot is recomputed from its key on the rare walk past it, so that only key and entry stay live.
+template <int MODE>
+__global__ void __launch_bounds__(256, 8) join_probe_packed_kernel(const long long* __restrict__ keys, int64_t tiles, const ulonglong2* __restrict__ packed,
+                                                                   unsigned int mask, unsigned long long kmin, int shift, int special, void* __restrict__ dst, int elem,
+                                                                   unsigned int* __restrict__ match_bits, unsigned long long* __restrict__ match_count)
+{
+    constexpr int ROWS = 2;
+    unsigned int matched = 0;
+    for (unsigned int t = blockIdx.x; t < (unsigned int)tiles; t += gridDim.x) {
+#pragma unroll 1
+        for (int h = 0; h < 4; h += ROWS) {
+            const unsigned int base = t * 1024u + h * 256u + threadIdx.x;
+            unsigned long long k[ROWS];
+            ulonglong2 s[ROWS];
+#pragma unroll
+            for (int j = 0; j < ROWS; j++) k[j] = (unsigned long long)__ldg(keys + base + j * 256);
+#pragma unroll
+            for (int j = 0; j < ROWS; j++) s[j] = __ldg(packed + (k[j] == EMPTY_KEY ? mask + 1u : lean_slot<MODE>(k[j], mask, kmin, shift)));
+#pragma unroll
+            for (int j = 0; j < ROWS; j++) {
+                if (s[j].x != k[j] && s[j].x != EMPTY_KEY) {            // the key left its home slot (INT64_MIN's entry always matches)
+                    unsigned int p = lean_slot<MODE>(k[j], mask, kmin, shift);
+                    do {
+                        p = lean_next<MODE>(p, (unsigned int)k[j] & 7u, mask);
+                        s[j] = __ldg(packed + p);
+                    } while (s[j].x != k[j] && s[j].x != EMPTY_KEY);
+                }
+                const bool hit = s[j].x == k[j] && (k[j] != EMPTY_KEY || special);
+                matched += match_bits_word(match_bits, t, h + j, hit);
+                const unsigned long long v = hit ? s[j].y : 0ULL;
+                const unsigned int i = base + j * 256;
+                switch (elem) {
+                    case 8: ((unsigned long long*)dst)[i] = v; break;
+                    case 4: ((unsigned int*)dst)[i] = (unsigned int)v; break;
+                    case 2: ((unsigned short*)dst)[i] = (unsigned short)v; break;
+                    default: ((unsigned char*)dst)[i] = (unsigned char)v; break;
+                }
+            }
+        }
+    }
+    if ((threadIdx.x & 31) == 0 && matched) atomicAdd(match_count, (unsigned long long)matched);
+}
+
+static int launch_packed(tgpu_ctx* ctx, const JoinGeom& geo, const long long* keys, int64_t tiles, const PackedSlot* packed, int special, void* dst, int elem,
+                         unsigned int* match_bits, unsigned long long* matches)
+{
+    const unsigned int mask32 = (unsigned int)geo.mask;
+    const ulonglong2* table = (const ulonglong2*)packed;
+    if (geo.mode == 2) {
+        auto k = join_probe_packed_kernel<2>;
+        TG_LAUNCH(ctx, k, lean_grid(ctx, k, tiles), 256, 0, keys, tiles, table, mask32, geo.kmin, geo.shift, special, dst, elem, match_bits, matches);
+    }
+    else if (geo.mode == 1) {
+        auto k = join_probe_packed_kernel<1>;
+        TG_LAUNCH(ctx, k, lean_grid(ctx, k, tiles), 256, 0, keys, tiles, table, mask32, 0ULL, 0, special, dst, elem, match_bits, matches);
+    }
+    else {
+        auto k = join_probe_packed_kernel<0>;
+        TG_LAUNCH(ctx, k, lean_grid(ctx, k, tiles), 256, 0, keys, tiles, table, mask32, 0ULL, 0, special, dst, elem, match_bits, matches);
+    }
+    return TGPU_OK;
 }
 
 // build payload re-laid out in SLOT order (one pass at build time): the fused probe then reads the payload right next
@@ -1037,7 +952,8 @@ struct tgpu_lookup {
     DevPage store;                      // key column first, then build output columns
     int32_t num_output = 0;
     std::vector<DevBuf> by_slot;        // build output columns in table-slot order (fused probe fast path)
-    DevBuf wide;                        // WideSlot[capacity + 1]: slots with the payload of their head row (<= 2 build output columns)
+    DevBuf wide;                        // WideSlot[capacity + 1]: slots with the payload of their head row (2 build output columns)
+    DevBuf packed;                      // PackedSlot[capacity + 1]: key + payload of the head row (1 build output column; no by_slot, no wide then)
     bool generic = false;               // keyed by row hash + verification against build_keys
     int attempts = 1;                   // generic only: hash functions the build needed (> 1 iff two keys shared a 64-bit hash)
     std::vector<DevColumn> build_keys;  // generic only: the real key columns of the build side
@@ -1115,7 +1031,7 @@ int lookup_positions(tgpu_ctx* ctx, const tgpu_lookup* lk, const DevColumn& key,
         if (tiles > 0) {
             GatherCols none;
             memset(&none, 0, sizeof(none));
-            TG_TRY(launch_lean<false>(ctx, lk->geo, (const long long*)key.data, tiles, (const int4*)table, lk->special_head, d_out, none, (unsigned long long*)nullptr));
+            TG_TRY(launch_lean<false>(ctx, lk->geo, (const long long*)key.data, tiles, (const int4*)table, lk->special_head, d_out, none, nullptr, nullptr));
             done = tiles * 1024;
         }
     }
@@ -1465,7 +1381,15 @@ struct JoinBuildOp : tgpu_op {
         bool slot_payload = !getenv("TGPU_JOIN_PAYLOAD_BY_ROW") && rows > 0 && lk->num_output > 0 && lk->num_output <= 4;
         for (int32_t b = 0; b < lk->num_output && slot_payload; b++)
             slot_payload = lk->store.cols[1 + b].elem_size() > 0 && lk->store.cols[1 + b].elem_size() <= 8 && !lk->store.cols[1 + b].validity;
-        if (slot_payload) {
+        // one output column: key and payload share a 16-byte entry, which replaces both the slot-ordered payload and the wide table
+        const bool packed = slot_payload && lk->num_output == 1 && !lk->has_dups && !lk->generic && cap + 1 < (1LL << 31);
+        if (packed) {
+            const DevColumn& c = lk->store.cols[1];
+            TG_TRY(lk->packed.alloc(ctx, (size_t)(cap + 1) * sizeof(PackedSlot)));
+            TG_LAUNCH(ctx, join_packed_table_kernel, tg_grid(ctx, cap + 1, 1024, 8), 256, 0, lk->table.as<JoinSlot>(), cap, lk->special_head, c.data, c.elem_size(),
+                      lk->packed.as<PackedSlot>());
+        }
+        else if (slot_payload) {
             lk->by_slot.resize(lk->num_output);
             for (int32_t b = 0; b < lk->num_output; b++) {
                 const DevColumn& c = lk->store.cols[1 + b];
@@ -1474,7 +1398,7 @@ struct JoinBuildOp : tgpu_op {
                           c.elem_size(), lk->by_slot[b].p);
             }
         }
-        if (slot_payload && lk->num_output <= 2 && !lk->has_dups && !lk->generic && cap + 1 < (1LL << 31) && !getenv("TGPU_JOIN_NO_WIDE")) {
+        if (slot_payload && !packed && lk->num_output <= 2 && !lk->has_dups && !lk->generic && cap + 1 < (1LL << 31) && !getenv("TGPU_JOIN_NO_WIDE")) {
             TG_TRY(lk->wide.alloc(ctx, (size_t)(cap + 1) * sizeof(WideSlot)));
             const DevColumn& c0 = lk->store.cols[1];
             const DevColumn* c1 = lk->num_output > 1 ? &lk->store.cols[2] : nullptr;
@@ -1512,7 +1436,7 @@ struct JoinProbeOp : tgpu_op {
     struct Deferred {
         bool active = false;
         DevPage in;
-        std::shared_ptr<DevBuf> jp;
+        std::shared_ptr<DevBuf> match_bits;     // bit i = probe row i matched (match_bits_word)
         std::vector<DevColumn> built;
         int64_t n = 0;
     } deferred;
@@ -1543,8 +1467,10 @@ struct JoinProbeOp : tgpu_op {
             const DevColumn& c = lookup->store.cols[1 + b];
             if (c.elem_size() == 0 || c.elem_size() > 8 || c.validity) return TGPU_OK;      // (the fused gather moves 1 / 2 / 4 / 8-byte payloads)
         }
-        auto jp = std::make_shared<DevBuf>();
-        TG_TRY(jp->alloc(ctx, (size_t)n * 4));
+        // one 32-bit word per 32 rows of every (possibly partial) 1024-row tile: each word is written by a probe kernel
+        auto bits = std::make_shared<DevBuf>();
+        TG_TRY(bits->alloc(ctx, (size_t)((n + 1023) / 1024) * 128));
+        unsigned int* d_bits = bits->as<unsigned int>();
         GatherCols g;
         memset(&g, 0, sizeof(g));
         g.count = lookup->num_output;
@@ -1564,34 +1490,38 @@ struct JoinProbeOp : tgpu_op {
         if (!match_counter.p) TG_TRY(match_counter.alloc(ctx, 16));       // [0] matches of the page, [1] (int) layout choice of the page
         unsigned long long* d_matches = match_counter.as<unsigned long long>();
         TG_CUDA(ctx, cudaMemsetAsync(d_matches, 0, 16, ctx->stream));     // no matches yet; layout choice 0 = the 16-byte slots
-        constexpr int ROWS = 4;
-        int grid = tg_grid(ctx, n, 256 * ROWS, 8);
-        auto k_fast = join_probe_gather_kernel<ROWS, true>;
-        auto k_any = join_probe_gather_kernel<ROWS, false>;
+        auto k_fast = join_probe_gather_kernel<true>;
+        auto k_any = join_probe_gather_kernel<false>;
         const JoinSlot* table = lookup->table.as<JoinSlot>();
         TG_TIMED_BEGIN(ctx);
         int64_t done = 0;
         bool fast = key.type == TGPU_INT64 && !key.validity;
         if (fast && !getenv("TGPU_JOIN_GENERIC_KERNELS")) {
             int64_t tiles = n / 1024;
-            if (tiles > 0) {
+            if (tiles > 0 && lookup->packed.p) {
+                // one output column: the packed table, whatever the page's key locality
+                TG_TRY(launch_packed(ctx, lookup->geo, (const long long*)key.data, tiles, lookup->packed.as<PackedSlot>(), lookup->special_head >= 0 ? 1 : 0, g.dst[0],
+                                     g.elem[0], d_bits, d_matches));
+                done = tiles * 1024;
+            }
+            else if (tiles > 0) {
                 // TGPU_JOIN_WIDE = always | never | auto (default): auto lets the page's key locality decide whenever the wide layout is the
                 // bigger one (payload cells < 16 bytes); with 16 bytes of payload the two layouts hold the same bytes and wide always wins
                 const char* we = getenv("TGPU_JOIN_WIDE");
                 int payload_bytes = 0;
                 for (int c = 0; c < g.count; c++) payload_bytes += g.elem[c];
-                const bool have_wide = lookup->wide.p && !getenv("TGPU_JOIN_NO_WIDE") && !getenv("TGPU_JOIN_SPAN") && !(we && !strcmp(we, "never"));
+                const bool have_wide = lookup->wide.p && !getenv("TGPU_JOIN_NO_WIDE") && !(we && !strcmp(we, "never"));
                 const bool always = have_wide && ((we && !strcmp(we, "always")) || payload_bytes >= 16 || !g.by_slot);
                 if (always)
-                    TG_TRY(launch_wide(ctx, lookup->geo, (const long long*)key.data, tiles, lookup->wide.as<WideSlot>(), lookup->special_head, jp->as<int>(), g, d_matches, nullptr));
+                    TG_TRY(launch_wide(ctx, lookup->geo, (const long long*)key.data, tiles, lookup->wide.as<WideSlot>(), lookup->special_head, g, d_bits, d_matches, nullptr));
                 else if (have_wide) {
                     int* d_choice = (int*)(d_matches + 1);
                     TG_TRY(launch_locality(ctx, lookup->geo, (const long long*)key.data, tiles, d_choice));
-                    TG_TRY(launch_lean<true>(ctx, lookup->geo, (const long long*)key.data, tiles, (const int4*)table, lookup->special_head, jp->as<int>(), g, d_matches));
-                    TG_TRY(launch_wide(ctx, lookup->geo, (const long long*)key.data, tiles, lookup->wide.as<WideSlot>(), lookup->special_head, jp->as<int>(), g, d_matches, d_choice));
+                    TG_TRY(launch_lean<true>(ctx, lookup->geo, (const long long*)key.data, tiles, (const int4*)table, lookup->special_head, nullptr, g, d_bits, d_matches));
+                    TG_TRY(launch_wide(ctx, lookup->geo, (const long long*)key.data, tiles, lookup->wide.as<WideSlot>(), lookup->special_head, g, d_bits, d_matches, d_choice));
                 }
                 else
-                    TG_TRY(launch_lean<true>(ctx, lookup->geo, (const long long*)key.data, tiles, (const int4*)table, lookup->special_head, jp->as<int>(), g, d_matches));
+                    TG_TRY(launch_lean<true>(ctx, lookup->geo, (const long long*)key.data, tiles, (const int4*)table, lookup->special_head, nullptr, g, d_bits, d_matches));
                 done = tiles * 1024;
             }
         }
@@ -1602,15 +1532,16 @@ struct JoinProbeOp : tgpu_op {
                 kr.data = (const char*)kr.data + done * 8;
                 for (int c = 0; c < gt.count; c++) gt.dst[c] = (char*)gt.dst[c] + done * gt.elem[c];
             }
-            int tgrid = tg_grid(ctx, n - done, 256 * ROWS, 8);
-            if (fast) TG_LAUNCH(ctx, k_fast, tgrid, 256, 0, kr, KEY_INT, n - done, table, lookup->geo, lookup->special_head, jp->as<int>() + done, gt, d_matches);
-            else TG_LAUNCH(ctx, k_any, tgrid, 256, 0, kr, key_kind_of(key.type), n - done, table, lookup->geo, lookup->special_head, jp->as<int>() + done, gt, d_matches);
+            // done is a multiple of 1024: the tail's tiles start on a word of the bitmap
+            int tgrid = tg_grid(ctx, n - done, 1024, 8);
+            if (fast) TG_LAUNCH(ctx, k_fast, tgrid, 256, 0, kr, KEY_INT, n - done, table, lookup->geo, lookup->special_head, gt, d_bits + done / 32, d_matches);
+            else TG_LAUNCH(ctx, k_any, tgrid, 256, 0, kr, key_kind_of(key.type), n - done, table, lookup->geo, lookup->special_head, gt, d_bits + done / 32, d_matches);
         }
         TG_TIMED_END(ctx);
         *handled = true;
         deferred.active = true;
         deferred.in = std::move(in);
-        deferred.jp = jp;
+        deferred.match_bits = bits;
         deferred.built = std::move(built);
         deferred.n = n;
         return TGPU_OK;
@@ -1654,7 +1585,7 @@ struct JoinProbeOp : tgpu_op {
     {
         deferred.active = false;
         DevPage in = std::move(deferred.in);
-        std::shared_ptr<DevBuf> jp = std::move(deferred.jp);
+        std::shared_ptr<DevBuf> bits = std::move(deferred.match_bits);
         std::vector<DevColumn> built = std::move(deferred.built);
         const int64_t n = deferred.n;
         const bool outer = join_type == TGPU_JOIN_PROBE_OUTER;     // (tracking join types never take the fast path)
@@ -1667,30 +1598,24 @@ struct JoinProbeOp : tgpu_op {
             // (LookupJoinPageBuilder.build :144-150 "outputProbeBlocksDirectly")
             outp.rows = n;
             for (int32_t ch : output_channels) outp.cols.push_back(in.cols[ch]);
-            std::shared_ptr<DevBuf> validity;
-            if (matches < n) {
-                validity = std::make_shared<DevBuf>();
-                TG_TRY(validity->alloc(ctx, (size_t)((n + 7) / 8)));
-                TG_LAUNCH(ctx, join_match_validity_kernel, tg_grid(ctx, (n + 7) / 8, 256, 8), 256, 0, jp->as<int>(), n, validity->as<uint8_t>());
-            }
+            // PROBE_OUTER with misses: the match bitmap is the build columns' validity
             for (auto& c : built) {
-                if (validity) { c.own_validity = validity; c.validity = validity->as<uint8_t>(); }
+                if (matches < n) { c.own_validity = bits; c.validity = bits->as<uint8_t>(); }
                 outp.cols.push_back(std::move(c));
             }
         }
         else {
             if (matches == 0) return TGPU_OK;
-            // compact the matched rows (stable): selection list, then sequential-read gathers
-            DevBuf flags, sel, tmp;
-            TG_TRY(flags.alloc(ctx, (size_t)n));
+            // compact the matched rows (stable): selection list from the match bitmap, then sequential-read gathers
+            DevBuf sel, tmp;
             TG_TRY(sel.alloc(ctx, (size_t)n * 4));
-            TG_LAUNCH(ctx, join_match_flags_kernel, tg_grid(ctx, n, 1024, 8), 256, 0, jp->as<int>(), n, flags.as<uint8_t>());
             long long* d_count = (long long*)(ctx->d_scratch + 14);
             size_t tmp_bytes = 0;
             thrust::counting_iterator<int32_t> iota(0);
-            cub::DeviceSelect::Flagged(nullptr, tmp_bytes, iota, flags.as<uint8_t>(), sel.as<int32_t>(), d_count, (int)n, ctx->stream);
+            const MatchBit matched{bits->as<unsigned int>()};
+            cub::DeviceSelect::If(nullptr, tmp_bytes, iota, sel.as<int32_t>(), d_count, (int)n, matched, ctx->stream);
             TG_TRY(tmp.alloc(ctx, tmp_bytes));
-            TG_CUDA(ctx, cub::DeviceSelect::Flagged(tmp.p, tmp_bytes, iota, flags.as<uint8_t>(), sel.as<int32_t>(), d_count, (int)n, ctx->stream));
+            TG_CUDA(ctx, cub::DeviceSelect::If(tmp.p, tmp_bytes, iota, sel.as<int32_t>(), d_count, (int)n, matched, ctx->stream));
             outp.rows = matches;
             for (int32_t ch : output_channels) {
                 DevColumn c;
@@ -2039,7 +1964,7 @@ extern "C" int64_t tgpu_lookup_memory_bytes(const tgpu_lookup* lookup)
     if (!lookup) return 0;
     int64_t b = (int64_t)lookup->table.bytes + (int64_t)lookup->links.bytes + lookup->store.memory_bytes();
     for (auto& s : lookup->by_slot) b += (int64_t)s.bytes;
-    b += (int64_t)lookup->wide.bytes;
+    b += (int64_t)lookup->wide.bytes + (int64_t)lookup->packed.bytes;
     return b;
 }
 
